@@ -2,6 +2,7 @@
 """bench.py — kriged grid points / second of the B200 backend='cuda' execute() path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--configs cfg1,cfg3,...|none]
+                    [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[1], SURVEY.md §8d cfg2): OrdinaryKriging 2-D, N=5000 random-scatter
 data (seed 1002), 1000x1000 grid, exponential variogram [1.0, 300, 0.05], fp64 (DMMA kernel).
@@ -18,6 +19,11 @@ and re-inverts on every call, ok.py:847,663 — so does every timed step here; n
           covariance-form triangular kernel actually issues (~ n^2 (1 + 256/n) per point).
   cpu_baseline : the oracle port of the reference's inverse x RHS path (oracle/krige_oracle.py) on the box's
           host cores (BLAS threads pinned to the core count), on a bounded sample of the same grid.
+
+--dump-outputs DIR writes what the last timed headline step computed, the whole 1000x1000 grid of kriged values
+and kriging variances, to DIR/zvalues.npy and DIR/sigmasq.npy (float64, shape (ny, nx) as execute('grid') returns
+them; 16 MB in all). The inputs are seeded, so two builds run with the same arguments can be compared output for
+output.
 
 N>1 (torchrun, one rank per GPU): rank 0 factors, one NCCL broadcast ships the factor blob, every rank kriges a
 contiguous slice of the SAME 1000x1000 grid (strong scaling: the headline `value`); the weak-scaling variant
@@ -353,9 +359,25 @@ def oracle_parity(ctx, cfg, model, xyz, val, axes, z_loc, ss_loc, first, count, 
     return out
 
 
-def bench_config(ctx, name, steps, warmup, e2e_steps, weak=False, dtype=None, parity=True, fatal_parity=False):
+def gather_grid(ctx, d_out, count, sizes):
+    """(z, sigma^2) of every rank's slice of the grid, as host arrays of the grid's shape (slowest axis first) on
+    rank 0; (None, None) on the other ranks."""
+    part = d_out[:2 * count].view(2, count).cpu().numpy()
+    parts = [part]
+    if ctx.world > 1:
+        parts = [None] * ctx.world
+        ctx.dist.all_gather_object(parts, part)
+    if ctx.rank != 0:
+        return None, None
+    zs = np.concatenate(parts, axis=1)
+    return zs[0].reshape(sizes[::-1]), zs[1].reshape(sizes[::-1])
+
+
+def bench_config(ctx, name, steps, warmup, e2e_steps, weak=False, dtype=None, parity=True, fatal_parity=False,
+                 outputs=None):
     """Time one BASELINE config on the ranks of this launch. Device-resident step (factor + krige this rank's
-    contiguous slice, outputs left in HBM) and end-to-end step (public API, host buffers). Max over ranks."""
+    contiguous slice, outputs left in HBM) and end-to-end step (public API, host buffers). Max over ranks.
+    `outputs` (a dict) receives the grid the last timed device-resident step computed (gather_grid)."""
     import pykrige_b200 as pk  # noqa: F401
     from pykrige_b200 import multigpu
     torch, dist = ctx.torch, ctx.dist
@@ -415,6 +437,8 @@ def bench_config(ctx, name, steps, warmup, e2e_steps, weak=False, dtype=None, pa
         step_dev()
     h.reset_counters()
     ms_dev = timed(ctx, step_dev, steps)
+    if outputs is not None:
+        outputs["zvalues"], outputs["sigmasq"] = gather_grid(ctx, d_out, count, sizes)
     tm = h.timings()
     launches = torch.tensor([tm["launches"]], dtype=torch.float64, device=ctx.dev)
     if ctx.world > 1:
@@ -516,9 +540,15 @@ def run_ours(args):
     # ---- headline: cfg2, fixed 1000x1000 grid split over the ranks (strong scaling) ----
     sampler = ClockSampler(local)
     sampler.start()
-    head, cfg2 = bench_config(ctx, "cfg2", args.steps, args.warmup, args.steps, parity=True, fatal_parity=True)
+    outputs = {} if args.dump_outputs else None
+    head, cfg2 = bench_config(ctx, "cfg2", args.steps, args.warmup, args.steps, parity=True, fatal_parity=True,
+                              outputs=outputs)
     sampler.stop_flag = True
     sampler.join(timeout=2.0)
+    if outputs is not None and ctx.rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
 
     extra = {}
     wanted = [] if args.configs == "none" else [c for c in args.configs.split(",") if c]
@@ -607,7 +637,13 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--configs", default="cfg1,cfg3,cfg4,cfg5",
                     help="other BASELINE configs to run after the headline (comma list, or 'none')")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the grid the last timed headline step computed to DIR/{zvalues,sigmasq}.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

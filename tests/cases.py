@@ -24,6 +24,19 @@ def synth_points(seed, m, dim, data_xyz, box=(1000.0, 1000.0, 250.0), n_hits=16)
     return np.vstack([pts, hits])
 
 
+# seeded inputs of the comparisons with the reference's compiled twins (golden/make_golden_native.py -> ref_native.npz):
+# name -> (seed, data points, query points, dim)
+NATIVE_INPUTS = {"global2d": (11, 300, 200, 2), "window2d": (14, 400, 150, 2), "window3d": (15, 400, 150, 3),
+                 "cuda2d": (2024, 1500, 2000, 2)}
+
+
+def native_inputs(name):
+    """(data coordinates, values, query points) of NATIVE_INPUTS[name]."""
+    seed, n, m, dim = NATIVE_INPUTS[name]
+    xyz, val = synth_data(seed, n, dim)
+    return xyz, val, synth_points(seed, m, dim, xyz)
+
+
 # functional drift terms by name (callables cannot be stored in fixtures)
 FUNCS = {
     "fx": lambda x, y: x,

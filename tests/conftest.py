@@ -63,6 +63,12 @@ def ref_ctor():
     return np.load(os.path.join(GOLDEN, "ref_ctor.npz"))
 
 
+@pytest.fixture(scope="session")
+def ref_native():
+    """Outputs of the reference's compiled cok.pyx twins on cases.NATIVE_INPUTS (make_golden_native.py)."""
+    return np.load(os.path.join(GOLDEN, "ref_native.npz"))
+
+
 def assert_parity(out, ref, R, what=""):
     """SURVEY.md §8(d): allclose(out, ref, rtol=R, atol=R*max|ref|)."""
     out = np.asarray(np.ma.getdata(out), dtype=np.float64)

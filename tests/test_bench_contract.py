@@ -1,9 +1,15 @@
-"""CPU test of the bench.py contract for the reference arm (`--impl reference`): one JSON line on stdout with
-the keys the driver reads; non-zero ranks print nothing."""
+"""The bench.py contract. Reference arm (`--impl reference`, CPU): one JSON line on stdout with the keys a reader of
+the result needs; non-zero ranks print nothing. CUDA arm (gpu): `--dump-outputs` writes the last timed step's grid."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
+
+import cases
+from conftest import assert_parity
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -30,3 +36,28 @@ def test_reference_arm_prints_one_json_line():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference"],
                          capture_output=True, text=True, env=env, timeout=60)
     assert out.returncode == 0 and out.stdout.strip() == ""
+
+
+@pytest.mark.gpu
+def test_ours_arm_dumps_the_last_timed_step(tmp_path):
+    """`--dump-outputs DIR`: the headline grid of the last timed step as (ny, nx) float64 arrays, in execute('grid')
+    orientation (checked against the CPU oracle on a few cells); `--steps` is the number of timed steps reported."""
+    from oracle import krige_oracle as ko
+    env = dict(os.environ, RANK="0", WORLD_SIZE="1")
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1",
+                          "--configs", "none", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, env=env, timeout=1200)
+    assert out.returncode == 0, out.stderr[-2000:]
+    lines = [ln for ln in out.stdout.splitlines() if ln.strip()]
+    assert len(lines) == 1 and json.loads(lines[0])["steps"] == 2
+    z, ss = np.load(tmp_path / "zvalues.npy"), np.load(tmp_path / "sigmasq.npy")
+    assert z.shape == ss.shape == (1000, 1000) and z.dtype == ss.dtype == np.float64
+    assert sorted(p.name for p in tmp_path.iterdir()) == ["sigmasq.npy", "zvalues.npy"]
+    xyz, val = cases.synth_data(1002, 5000, 2)
+    gx = gy = np.linspace(0.0, 1000.0, 1000)
+    rng = np.random.default_rng(5)
+    iy, ix = rng.integers(0, 1000, 32), rng.integers(0, 1000, 32)
+    zo, so = ko.krige(xyz, val, "exponential", ko.stored_parameters("exponential", [1.0, 300.0, 0.05]),
+                      np.column_stack([gx[ix], gy[iy]]))
+    assert_parity(z[iy, ix], zo, 1e-5, "z")
+    assert_parity(ss[iy, ix], so, 1e-5, "ss")

@@ -181,39 +181,33 @@ def test_oracle_pseudo_inverse_known_answer(ptype):
     assert np.isclose(z[0], 2.0)
 
 
-# ---- the reference's compiled native twins (oracle/_ref, built by oracle/build_ref.py) ----------------
-def _native():
-    from oracle import ref_native
-    if not ref_native.available():
-        pytest.skip("oracle/_ref is not built (python oracle/build_ref.py, needs /root/reference)")
-    return ref_native
+# ---- the reference's compiled native twins (outputs stored by golden/make_golden_native.py) -----------
+def _native_inputs(name, ref_native):
+    xyz, val, pts = cases.native_inputs(name)
+    assert_allclose([xyz.sum(), val.sum(), pts.sum()], ref_native[name + "/fp"], rtol=1e-12)
+    return xyz, val, pts
 
 
 @pytest.mark.parametrize("model", ["linear", "power", "gaussian", "exponential", "spherical"])
-def test_oracle_matches_compiled_reference_twin(model):
+def test_oracle_matches_compiled_reference_twin(model, ref_native):
     """The numpy restatement vs the reference's own compiled `_c_exec_loop` (cok.pyx:14-96), same inputs."""
-    rn = _native()
-    xyz, val = cases.synth_data(11, 300, 2)
-    pts = cases.synth_points(11, 200, 2, xyz)
+    xyz, val, pts = _native_inputs("global2d", ref_native)
     stored = ko.stored_parameters(model, cases.MODELS[model])
     for exact in (True, False):
-        z, ss = rn.exec_loop(xyz, pts, val, model, stored, exact_values=exact)
+        key = "global2d/%s/%s" % (model, "exact" if exact else "inexact")
         zo, so = ko.krige(xyz, val, model, stored, pts, exact_values=exact)
-        assert_parity(zo, z, 1e-8, "z")
-        assert_parity(so, ss, 1e-8, "ss")
+        assert_parity(zo, ref_native[key + "/z"], 1e-8, "z")
+        assert_parity(so, ref_native[key + "/ss"], 1e-8, "ss")
 
 
-def test_oracle_moving_window_matches_compiled_reference_twin():
+def test_oracle_moving_window_matches_compiled_reference_twin(ref_native):
     """... and `_c_exec_loop_moving_window` (cok.pyx:98-193), 2-D and 3-D."""
-    rn = _native()
-    for dim, k in ((2, 8), (3, 12)):
-        xyz, val = cases.synth_data(12 + dim, 400, dim)
-        pts = cases.synth_points(12 + dim, 150, dim, xyz)
+    for name, k in (("window2d", 8), ("window3d", 12)):
+        xyz, val, pts = _native_inputs(name, ref_native)
         stored = ko.stored_parameters("exponential", [1.0, 150.0, 0.05])
-        z, ss = rn.exec_loop_moving_window(xyz, pts, val, "exponential", stored, k)
         zo, so = ko.krige(xyz, val, "exponential", stored, pts, n_closest_points=k)
-        assert_parity(zo, z, 1e-9, "z")
-        assert_parity(so, ss, 1e-9, "ss")
+        assert_parity(zo, ref_native["%s/k%d/z" % (name, k)], 1e-9, "z")
+        assert_parity(so, ref_native["%s/k%d/ss" % (name, k)], 1e-9, "ss")
 
 
 # ---- variogram_model='custom' ---------------------------------------------------------------------------

@@ -737,29 +737,23 @@ def test_whole_chain_scenarios_match_reference(pk, sc, ref_scenarios, ref_golden
                         atol=1e-5 * np.abs(ref_scenarios[sc["name"] + "/epsilon"]).max())
 
 
-# ---- straight against the reference's compiled native code (oracle/_ref travels to the GPU box) ---------
-def test_cuda_matches_compiled_reference_twins(pk):
-    """backend='cuda' vs the reference's own `_c_exec_loop` / `_c_exec_loop_moving_window` (lib/cok.pyx,
-    compiled by oracle/build_ref.py) on fresh seeded inputs — no committed fixture in between."""
-    from oracle import ref_native as rn, krige_oracle as ko
-    if not rn.available():
-        pytest.skip("oracle/_ref is not built")
-    xyz, val = cases.synth_data(2024, 1500, 2)
-    pts = cases.synth_points(2024, 2000, 2, xyz)
+# ---- straight against the reference's compiled native code (outputs stored by golden/make_golden_native.py) ----
+def test_cuda_matches_compiled_reference_twins(pk, ref_native):
+    """backend='cuda' vs the reference's own `_c_exec_loop` / `_c_exec_loop_moving_window` (lib/cok.pyx) on
+    seeded inputs."""
+    xyz, val, pts = cases.native_inputs("cuda2d")
+    assert_allclose([xyz.sum(), val.sum(), pts.sum()], ref_native["cuda2d/fp"], rtol=1e-12)
     for model in ("exponential", "spherical", "linear"):
         params = cases.MODELS[model]
         m = pk.OrdinaryKriging(xyz[:, 0], xyz[:, 1], val, variogram_model=model, variogram_parameters=list(params))
         z, ss = m.execute("points", pts[:, 0], pts[:, 1], backend="cuda")
-        zr, sr = rn.exec_loop(xyz, pts, val, model, ko.stored_parameters(model, params))
-        assert_parity(z, zr, R64, model + " z vs cok._c_exec_loop")
-        assert_parity(ss, sr, R64, model + " ss vs cok._c_exec_loop")
+        assert_parity(z, ref_native["cuda2d/%s/z" % model], R64, model + " z vs cok._c_exec_loop")
+        assert_parity(ss, ref_native["cuda2d/%s/ss" % model], R64, model + " ss vs cok._c_exec_loop")
     m = pk.OrdinaryKriging(xyz[:, 0], xyz[:, 1], val, variogram_model="exponential",
                            variogram_parameters=[1.0, 150.0, 0.05])
     z, ss = m.execute("points", pts[:, 0], pts[:, 1], backend="cuda", n_closest_points=16)
-    zr, sr = rn.exec_loop_moving_window(xyz, pts, val, "exponential",
-                                        ko.stored_parameters("exponential", [1.0, 150.0, 0.05]), 16)
-    assert_parity(z, zr, R64, "knn z vs cok._c_exec_loop_moving_window")
-    assert_parity(ss, sr, R64, "knn ss vs cok._c_exec_loop_moving_window")
+    assert_parity(z, ref_native["cuda2d/k16/z"], R64, "knn z vs cok._c_exec_loop_moving_window")
+    assert_parity(ss, ref_native["cuda2d/k16/ss"], R64, "knn ss vs cok._c_exec_loop_moving_window")
 
 
 # ---- BASELINE configs 3, 4, 5 at their full data sizes: size-independent properties + oracle subsample ----
