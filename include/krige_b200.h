@@ -56,7 +56,9 @@ extern "C" {
 #define KB200_VG_TABLE        6  /* 'custom' / GSTools callables (ok.py:224-253): tabulated by the host, see kb200_set_variogram_table; no params */
 
 /* ---- arithmetic of the big contraction ---------------------------------- */
-#define KB200_F64 0
+#define KB200_F64 0   /* fp64 contraction: with a positive definite covariance form and 512 <= n <= 65535 on the INT8
+                         tensor cores with 8 exact slices (55 bits, as accurate as the fp64 product), else on the fp64
+                         DMMA tensor cores (small n, pseudo_inv, the indefinite general path) */
 #define KB200_F32 1   /* factorisation stays fp64; contraction in 3xTF32 on tcgen05 (fp32-class accuracy) */
 #define KB200_F64X 2  /* fp64-class contraction on the INT8 tensor cores: error-free slicing into 6 signed slices (41 bits),
                          exact int32 accumulation (tcgen05 kind::i8), exact int64 recombination; agrees with KB200_F64
@@ -282,6 +284,7 @@ int kb200_set_stream(kb200_handle h, void* cuda_stream);
  *  [4] solve kernel (sum over chunks)  [5] finalize (sum)  [6] h2d  [7] d2h
  *  [8] knn search  [9] knn local solve
  *  [10] solve-kernel launches  [11] total kernel launches since the last kb200_reset_counters
+ *  [12] slices of the INT8 contraction kernel of the current problem (0 = fp64 DMMA or 3xTF32 kernel)
  * Returns the number of entries written (<= n).
  */
 int  kb200_last_timings(kb200_handle h, double* ms, int n);

@@ -158,7 +158,7 @@ def _f64(a):
 
 
 TIMING_KEYS = ["assemble_ms", "cholesky_ms", "trtri_ms", "pack_dual_ms", "solve_ms", "finalize_ms",
-               "h2d_ms", "d2h_ms", "knn_search_ms", "knn_solve_ms", "solve_launches", "launches"]
+               "h2d_ms", "d2h_ms", "knn_search_ms", "knn_solve_ms", "solve_launches", "launches", "solve_slices"]
 
 
 class Handle:
@@ -334,8 +334,8 @@ class Handle:
 
     # -- instrumentation ------------------------------------------------------------------
     def timings(self):
-        buf = (ctypes.c_double * 12)()
-        n = self.lib.kb200_last_timings(self._h, buf, 12)
+        buf = (ctypes.c_double * len(TIMING_KEYS))()
+        n = self.lib.kb200_last_timings(self._h, buf, len(TIMING_KEYS))
         return {TIMING_KEYS[i]: buf[i] for i in range(n)}
 
     def reset_counters(self):

@@ -28,6 +28,26 @@ struct Src {
 // general (indefinite) path: blocked Gauss-Jordan unless KB200_GJ=scalar
 #define KB_GJ_DEFAULT_BLOCKED 1
 
+// dtype='float64' contraction: on the Cholesky path with KB_F64_I8_NMIN <= n <= KB_F64_I8_NMAX the INT8 slice kernel with
+// 8 exact slices (55 bits, as accurate as the fp64 product; solve_i8.cu), else the DMMA kernel (solve.cu). The int32
+// accumulators bound n (n * 8 * 64^2 < 2^31). Solve kernel, int8 over DMMA on a B200: 1.00x at n=256, 1.17x at 512,
+// 1.42x at 1024, 1.73x at 2048 (profiles/README.md, scripts/f64_route_timing.py).
+#define KB_F64_I8_SLICES 8
+#define KB_F64_I8_NMIN 512
+#define KB_F64_I8_NMAX 65535
+
+// Slice count of the contraction of a dtype='float64' problem (0 = DMMA). A function of the problem alone, never of the
+// prediction points, so that shards, chunks and devices all run the same kernel. KB200_F64_SOLVE=dmma | int8 overrides
+// the size rule; it is the cross-check and profiling switch of the tests and scripts, read when a problem is described.
+static int f64_route_slices(int64_t n, bool pinv) {
+    if (pinv || n > KB_F64_I8_NMAX) return 0;
+    if (const char* e = std::getenv("KB200_F64_SOLVE")) {
+        if (std::strcmp(e, "dmma") == 0) return 0;
+        if (std::strcmp(e, "int8") == 0) return KB_F64_I8_SLICES;
+    }
+    return n >= KB_F64_I8_NMIN ? KB_F64_I8_SLICES : 0;
+}
+
 struct DevBuf {
     void* p = nullptr; size_t cap = 0;
     cudaError_t reserve(size_t bytes) {
@@ -51,7 +71,7 @@ struct kb200_ctx {
     // description
     bool described = false, ready = false, knn_ready = false;
     bool factor_live = false;  // L (wC) and the forward solves (wF) of the ready problem are still in the workspace
-    int slices = 0;           // int8-slice dtypes: number of slices (6 / 5 / 4), else 0
+    int slices = 0;           // contraction on the INT8 slice kernel: number of slices (float64: 8; float64x*: 6 / 5 / 4), else 0
     int gform = 0;            // 1: general (indefinite) fallback, tiles hold the symmetric inverse
     int geo = 0;              // 1: coordinates_type='geographic' for the next problem description
     int pinv = 0;             // 1: pseudo_inv=True for the next problem description (global path only)
@@ -94,7 +114,7 @@ struct kb200_ctx {
     int k_ncells = 0;
 
     cudaEvent_t ev[16] = {};
-    double tm[12] = {};
+    double tm[13] = {};
     long long launches = 0, solve_launches = 0;
 };
 
@@ -187,7 +207,8 @@ extern "C" int kb200_last_timings(kb200_handle h, double* ms, int n) {
     if (!h || !ms) return KB200_EBADARG;
     h->tm[10] = (double)h->solve_launches;
     h->tm[11] = (double)h->launches;
-    int m = std::min(n, 12);
+    h->tm[12] = (double)h->slices;
+    int m = std::min(n, 13);
     for (int i = 0; i < m; ++i) ms[i] = h->tm[i];
     return m;
 }
@@ -268,6 +289,7 @@ static int describe(kb200_ctx* h, bool knn_only, int dim, int dtype, int64_t n,
     if (n_dev && dim != 2) return fail(h, KB200_EUNSUPPORTED, "point_log / external_Z drift terms are two-dimensional (uk.py)");
     h->n_dev = n_dev;
     h->slices = dtype == KB200_F64X ? 6 : dtype == KB200_F64X5 ? 5 : dtype == KB200_F64X4 ? 4 : 0;
+    if (dtype == KB200_F64 && !knn_only) h->slices = f64_route_slices(n, h->pinv != 0);
 
     const int user_dim = dim;
     h->dim = h->geo ? KB_GEO : dim; h->dtype = dtype; h->n = (int)n; h->n_rl = n_rl; h->n_hd = n_hd;
@@ -365,13 +387,17 @@ static int describe(kb200_ctx* h, bool knn_only, int dim, int dtype, int64_t n,
     h->off_ay = o; o += align_up((size_t)h->n_pad * 8, 256);
     h->off_az = o; o += align_up((size_t)h->n_pad * 8, 256);
     h->off_tiles = o;
-    if (h->slices) {
-        o += (size_t)kbk_i8_total_tiles(h->slices, (int)n, h->na, nullptr) * kbk_i8_tile_bytes(h->slices);
-        o = align_up(o, 256);
-        h->off_rowscale = o; o += align_up((size_t)kbk_i8_rows(h->slices, (int)n, h->na) * sizeof(double), 256);
-    } else {
-        o += (size_t)off * KB_BM * KB_BK * esz;
+    // a float64 problem that may take the int8 route reserves room for both layouts: whether the Cholesky succeeds (else
+    // the general path packs fp64 tiles) is known only after the factorisation, and every rank sizes the blob alike
+    const int i8s = (dtype == KB200_F64) ? ((h->pinv || n > KB_F64_I8_NMAX) ? 0 : KB_F64_I8_SLICES) : h->slices;
+    size_t o8 = o;
+    if (i8s) {
+        o8 += (size_t)kbk_i8_total_tiles(i8s, (int)n, h->na, nullptr) * kbk_i8_tile_bytes(i8s);
+        o8 = align_up(o8, 256);
+        h->off_rowscale = o8; o8 += align_up((size_t)kbk_i8_rows(i8s, (int)n, h->na) * sizeof(double), 256);
     }
+    if (dtype == KB200_F64 || dtype == KB200_F32) o += (size_t)off * KB_BM * KB_BK * esz;
+    o = std::max(o, o8);
     h->blob_bytes = knn_only ? h->off_tiles : o;
     cudaSetDevice(h->device);
     CU(h, h->blob.reserve(h->blob_bytes));
@@ -391,7 +417,7 @@ extern "C" int kb200_describe_problem(kb200_handle h, int dim, int dtype, int64_
 extern "C" int64_t kb200_blob_bytes(kb200_handle h) { return (h && h->described) ? (int64_t)h->blob_bytes : 0; }
 extern "C" void* kb200_blob_ptr(kb200_handle h) { return (h && h->described) ? h->blob.p : nullptr; }
 
-// header layout (doubles): [0] magic, [1] c0, [2..18) shift, [18..34) scale
+// header layout (doubles): [0] magic, [1] c0, [2..18) shift, [18..34) scale, [34] gform, [35] slices
 static const double KB_MAGIC = 20260922.0;
 
 extern "C" int kb200_blob_commit(kb200_handle h) {
@@ -403,6 +429,7 @@ extern "C" int kb200_blob_commit(kb200_handle h) {
     if (hdr[0] != KB_MAGIC) return fail(h, KB200_ESTATE, "blob does not hold a factored problem");
     h->vg.c0 = hdr[1];
     h->gform = (int)hdr[34];
+    h->slices = (int)hdr[35];        // the kernel the factoring handle packed for
     for (int c = 0; c <= KB200_MAX_DRIFT; ++c) { h->ds.shift[c] = hdr[2 + c]; h->ds.scale[c] = hdr[18 + c]; }
     h->ready = true;
     return KB200_OK;
@@ -517,6 +544,7 @@ extern "C" int kb200_set_problem(kb200_handle h, int dim, int dtype, int64_t n,
                         "(the variogram is not valid in this dimension); use float64");
         }
         h->vg.c0 = c0_first;
+        h->slices = 0;                                  // fp64 quadratic-form tiles, DMMA kernel
         CU(h, cudaMemsetAsync(flag, 0, sizeof(int), st));
         CU(h, cudaEventRecord(h->ev[3], st));
         CU(h, kbk_assemble(h->dim, h->vg, nn, np, ld, ax, ay, az, h->wC.as<double>(), st)); ++launches;
@@ -564,7 +592,7 @@ extern "C" int kb200_set_problem(kb200_handle h, int dim, int dtype, int64_t n,
     ++launches;
     }
     double hdr[64] = {0};
-    hdr[0] = KB_MAGIC; hdr[1] = h->vg.c0; hdr[34] = (double)h->gform;
+    hdr[0] = KB_MAGIC; hdr[1] = h->vg.c0; hdr[34] = (double)h->gform; hdr[35] = (double)h->slices;
     for (int c = 0; c <= KB200_MAX_DRIFT; ++c) { hdr[2 + c] = h->ds.shift[c]; hdr[18 + c] = h->ds.scale[c]; }
     CU(h, cudaMemcpyAsync(blob, hdr, sizeof(hdr), cudaMemcpyHostToDevice, st));
     CU(h, cudaEventRecord(h->ev[6], st));

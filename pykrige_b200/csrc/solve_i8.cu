@@ -1,18 +1,19 @@
-// solve_i8.cu — K3 for dtype = KB200_F64X / F64X5 / F64X4: fp64-class accuracy of q_j = ||W c_j||^2 (DESIGN.md §3)
-// on the INT8 path of the 5th-generation tensor cores (tcgen05.mma kind::i8, exact int32 accumulation in TMEM).
+// solve_i8.cu — K3 on the INT8 path of the 5th-generation tensor cores (tcgen05.mma kind::i8, exact int32 accumulation
+// in TMEM): q_j = ||W c_j||^2 (DESIGN.md §3) for dtype = KB200_F64 (S = 8, the default fp64 route for
+// KB_F64_I8_NMIN <= n <= 65535 on the Cholesky path, api.cu) and KB200_F64X / F64X5 / F64X4 (S = 6 / 5 / 4).
 //
 // Error-free slicing (the "Ozaki scheme"): every row of W and every RHS column is scaled by a power of two
-// into (-1, 1) and cut into S signed slices of 6+7+...+7 bits (S = 6: 41 bits, 5: 34 bits, 4: 27 bits),
+// into (-1, 1) and cut into S signed slices of 6+7+...+7 bits (S = 8: 55 bits, 6: 41, 5: 34, 4: 27),
 //      x = 2^e * sum_s slice_s * 2^(-6-7s),   |slice_s| <= 64,
 // so that  W_rk c_k = 2^(ew_r + ec_j) * sum_{s,t} w_s c_t 2^(-12-7(s+t)).  All slice products with the
 // same d = s + t are summed EXACTLY in one int32 TMEM accumulator (|sum| <= n * (d+1) * 64^2 < 2^31 for
-// n <= 32512); pairs with d >= S are dropped (relative 2^-(7S+6) per term). The S accumulators are combined
-// exactly in int64 in the epilogue and converted to fp64 once. S = 6 agrees with the fp64 DMMA kernel to ~1e-10
-// (tests) at several times its rate; fewer slices trade bits for MMAs (S(S+1)/2 per k-stage: 21 / 15 / 10) and
-// operand bytes; dtype='float64' keeps the DMMA kernel as the default.
+// n <= 65535 at S = 8); pairs with d >= S are dropped (relative 2^-(7S+6) per term). The S accumulators are combined
+// exactly in int64 in the epilogue and converted to fp64 once. S = 8 is as accurate as the fp64 product it replaces
+// (tests/test_f64_int8_route.py); S = 6 agrees with the fp64 DMMA kernel to ~1e-10; fewer slices trade bits for MMAs
+// (S(S+1)/2 per k-stage: 36 / 21 / 15 / 10) and operand bytes.
 //
 // Orientation as in solve_tf32.cu: D[point][W row], M = 128 points (TMEM lanes), N = BN W rows per row block
-// with S * BN <= 512 TMEM columns (BN = 80 / 96 / 128: the RHS slices are re-read once per row block, so fewer
+// with S * BN <= 512 TMEM columns (BN = 64 / 80 / 96 / 128: the RHS slices are re-read once per row block, so fewer
 // slices also mean fewer re-reads), K = 32 per MMA; operands in the canonical no-swizzle K-major UMMA layout
 // (8-row x 16-byte core matrices, k-chunks 128 B apart, 8-row groups 256 B apart), one stage = 32 k = one MMA
 // k-step. The variogram model is a run-time switch here (phase G is < 10 % of the kernel), so that the slice
@@ -27,8 +28,8 @@
 #define I8_C_SLICE (I8_TM * I8_BK)            // 4 KB
 
 template <int S> struct I8Cfg {
-    static constexpr int BN = (S == 6) ? 80 : (S == 5) ? 96 : 128;     // S * BN <= 512 TMEM columns, BN % 16 == 0
-    static constexpr int STAGES = (S == 4) ? 6 : 5;
+    static constexpr int BN = (S == 8) ? 64 : (S == 6) ? 80 : (S == 5) ? 96 : 128;   // S * BN <= 512 TMEM columns, BN % 16 == 0
+    static constexpr int STAGES = (S == 8) ? 4 : (S == 4) ? 6 : 5;                 // S = 8: 4 x 48 KB stages
     static constexpr int W_SLICE = BN * I8_BK;
     static constexpr int W_BYTES = S * W_SLICE;
     static constexpr int C_BYTES = S * I8_C_SLICE;
@@ -76,6 +77,24 @@ __device__ __forceinline__ void i8_mma(uint32_t tmem_d, uint64_t da, uint64_t db
 __device__ __forceinline__ void i8_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];\n"
                  :: "r"(i8_smem_u32(bar)) : "memory");
+}
+
+// CW consecutive 32-bit TMEM columns of this thread's lane (CW = 8 or 16), waited for
+template <int CW>
+__device__ __forceinline__ void i8_tmem_ld(uint32_t taddr, uint32_t (&u)[CW]) {
+    if constexpr (CW == 16) {
+        asm volatile(
+            "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
+            "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];\n"
+            : "=r"(u[0]), "=r"(u[1]), "=r"(u[2]), "=r"(u[3]), "=r"(u[4]), "=r"(u[5]), "=r"(u[6]), "=r"(u[7]),
+              "=r"(u[8]), "=r"(u[9]), "=r"(u[10]), "=r"(u[11]), "=r"(u[12]), "=r"(u[13]), "=r"(u[14]), "=r"(u[15])
+            : "r"(taddr));
+    } else {
+        asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];\n"
+                     : "=r"(u[0]), "=r"(u[1]), "=r"(u[2]), "=r"(u[3]), "=r"(u[4]), "=r"(u[5]), "=r"(u[6]), "=r"(u[7])
+                     : "r"(taddr));
+    }
+    asm volatile("tcgen05.wait::ld.sync.aligned;\n" ::: "memory");
 }
 
 // S signed 7-bit digits of y = x * 2^-e (|y| < 1): x = 2^e * sum_s out[s] * 2^(-6-7s) + O(2^(e-7S)), out[s] in [-64, 64].
@@ -231,6 +250,7 @@ __global__ void __launch_bounds__(I8_THREADS, 1) solve_kernel_i8(const __grid_co
         // ---------------- generators: RHS column block -> S int8 slices per value, UMMA layout ----------------
         const int pl = (tid - 8 * 32) & (I8_TM - 1);       // 0..127: point within the tile
         const int ks = (tid - 8 * 32) >> 7;                // 0..1: k-stage parity handled by this thread
+        constexpr int KW = (S == 8) ? 8 : 16;              // k values sliced per store (S = 8: fewer live slice bytes)
         uint32_t it = 0;
         for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++it) {
             const int b = (int)(it & 1);
@@ -259,11 +279,11 @@ __global__ void __launch_bounds__(I8_THREADS, 1) solve_kernel_i8(const __grid_co
             for (int t = ks; t < nk; t += I8_GEN_THREADS / I8_TM) {
                 unsigned char* ct = sc + (size_t)t * C::C_BYTES;
 #pragma unroll 1
-                for (int kc = 0; kc < 2; ++kc) {           // two 16-byte k-chunks per stage
-                    signed char sl[16][S];
+                for (int kc = 0; kc < I8_BK / KW; ++kc) {  // KW-byte k-chunks per stage
+                    signed char sl[KW][S];
 #pragma unroll
-                    for (int kk = 0; kk < 16; ++kk) {
-                        const int k = t * I8_BK + kc * 16 + kk;
+                    for (int kk = 0; kk < KW; ++kk) {
+                        const int k = t * I8_BK + kc * KW + kk;
                         double c = 0.0;
                         if (pvalid && k < P.n) {
                             double d = kb_dist<DIM>(__ldg(P.ax + k), __ldg(P.ay + k), KB_HASZ(DIM) ? __ldg(P.az + k) : 0.0, px, py, pz);
@@ -271,15 +291,16 @@ __global__ void __launch_bounds__(I8_THREADS, 1) solve_kernel_i8(const __grid_co
                         }
                         i8_slice_scaled<S>(c, cscale, sl[kk]);
                     }
-                    const int off = (pl >> 3) * 256 + kc * 128 + (pl & 7) * 16;
+                    const int off = i8_off(pl, kc * KW);
 #pragma unroll
                     for (int s = 0; s < S; ++s) {
-                        uint32_t w[4];
+                        uint32_t w[KW / 4];
 #pragma unroll
-                        for (int q = 0; q < 4; ++q)
+                        for (int q = 0; q < KW / 4; ++q)
                             w[q] = (uint32_t)(uint8_t)sl[4 * q][s] | ((uint32_t)(uint8_t)sl[4 * q + 1][s] << 8) |
                                    ((uint32_t)(uint8_t)sl[4 * q + 2][s] << 16) | ((uint32_t)(uint8_t)sl[4 * q + 3][s] << 24);
-                        *reinterpret_cast<uint4*>(ct + s * I8_C_SLICE + off) = make_uint4(w[0], w[1], w[2], w[3]);
+                        if constexpr (KW == 16) *reinterpret_cast<uint4*>(ct + s * I8_C_SLICE + off) = make_uint4(w[0], w[1], w[2], w[3]);
+                        else *reinterpret_cast<uint2*>(ct + s * I8_C_SLICE + off) = make_uint2(w[0], w[1]);
                     }
                 }
             }
@@ -344,6 +365,7 @@ __global__ void __launch_bounds__(I8_THREADS, 1) solve_kernel_i8(const __grid_co
         }
     } else if (warp >= 4) {
         // ---------------- epilogue: thread = TMEM lane = prediction point ----------------
+        constexpr int CW = (S == 8) ? 8 : 16;               // TMEM columns per load (S = 8: H and L both live)
         const int pl = (warp & 3) * 32 + lane;
         const uint32_t t_addr = tmem_base + (((uint32_t)(warp & 3) * 32u) << 16);
         uint32_t gb = 0, it = 0;
@@ -356,31 +378,34 @@ __global__ void __launch_bounds__(I8_THREADS, 1) solve_kernel_i8(const __grid_co
                 i8_mbar_wait(tfull, (uint32_t)(gb & 1));
                 asm volatile("tcgen05.fence::after_thread_sync;\n" ::: "memory");
 #pragma unroll 1
-                for (int ch = 0; ch < C::BN / 16; ++ch) {
-                    // exact recombination: V = sum_d acc_d * 2^(7 (S-1-d)) fits in int64 (|acc_d| < 2^30, d = 0 has one
-                    // slice pair: < 2^27 * 2^35)
-                    long long V[16];
+                for (int ch = 0; ch < C::BN / CW; ++ch) {
+                    // exact recombination: V = sum_d acc_d * 2^(7 (S-1-d)).  S <= 6: V fits in int64 (|acc_d| < 2^30, d = 0
+                    // has one slice pair: < 2^27 * 2^35).  S = 8: |acc_0| <= n * 2^12 shifted by 2^49 can exceed int64, so
+                    // V = H * 2^28 + L with H = sum_{d<4} acc_d 2^(7 (3-d)), L = sum_{d>=4} acc_d 2^(7 (7-d)); for
+                    // n <= 65535 (|acc_d| < (d+1) 2^28) |H| < 2^50 and |L| < 2^52 are exact in int64 and in fp64, and
+                    // (double)H * 2^28 + (double)L rounds V once
+                    long long V[CW];
+                    double X[CW];
 #pragma unroll
-                    for (int j = 0; j < 16; ++j) V[j] = 0;
+                    for (int j = 0; j < CW; ++j) V[j] = 0;
 #pragma unroll
                     for (int d = 0; d < S; ++d) {
-                        uint32_t u[16];
-                        asm volatile(
-                            "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-                            "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];\n"
-                            : "=r"(u[0]), "=r"(u[1]), "=r"(u[2]), "=r"(u[3]), "=r"(u[4]), "=r"(u[5]), "=r"(u[6]), "=r"(u[7]),
-                              "=r"(u[8]), "=r"(u[9]), "=r"(u[10]), "=r"(u[11]), "=r"(u[12]), "=r"(u[13]), "=r"(u[14]), "=r"(u[15])
-                            : "r"(t_addr + (uint32_t)d * C::BN + (uint32_t)ch * 16u));
-                        asm volatile("tcgen05.wait::ld.sync.aligned;\n" ::: "memory");
+                        uint32_t u[CW];
+                        i8_tmem_ld<CW>(t_addr + (uint32_t)d * C::BN + (uint32_t)(ch * CW), u);
 #pragma unroll
-                        for (int j = 0; j < 16; ++j) V[j] = V[j] * 128 + (long long)(int)u[j];
+                        for (int j = 0; j < CW; ++j) V[j] = V[j] * 128 + (long long)(int)u[j];
+                        if (S == 8 && d == 3) {
+#pragma unroll
+                            for (int j = 0; j < CW; ++j) { X[j] = (double)V[j] * 268435456.0; V[j] = 0; }   // H * 2^28
+                        }
                     }
-                    const int r0 = J * C::BN + ch * 16;
+                    const int r0 = J * C::BN + ch * CW;
 #pragma unroll
-                    for (int j = 0; j < 16; ++j) {
+                    for (int j = 0; j < CW; ++j) {
                         const int r = r0 + j;
                         if (r < P.n + P.na) {
-                            const double x = (double)V[j] * (__ldg(P.rowscale + r) * pscale);
+                            const double v = (S == 8) ? X[j] + (double)V[j] : (double)V[j];
+                            const double x = v * (__ldg(P.rowscale + r) * pscale);
                             if (r < P.n) q += x * x;
                             else auxs[(r - P.n) * I8_TM + pl] = x;
                         }
@@ -409,8 +434,8 @@ template <int S> static size_t i8_smem_s() {
     return (size_t)I8Cfg<S>::STAGES * I8Cfg<S>::STAGE_BYTES + (size_t)KB_MAXAUX * I8_TM * sizeof(double) + 2 * I8_TM * sizeof(int) +
            (2 * I8Cfg<S>::STAGES + 6) * sizeof(uint64_t) + 64;
 }
-static int i8_bn(int S) { return S == 6 ? I8Cfg<6>::BN : S == 5 ? I8Cfg<5>::BN : I8Cfg<4>::BN; }
-bool kbk_i8_valid_slices(int S) { return S >= 4 && S <= 6; }
+static int i8_bn(int S) { return S == 8 ? I8Cfg<8>::BN : S == 6 ? I8Cfg<6>::BN : S == 5 ? I8Cfg<5>::BN : I8Cfg<4>::BN; }
+bool kbk_i8_valid_slices(int S) { return (S >= 4 && S <= 6) || S == 8; }
 int kbk_i8_nrb(int S, int n, int na) { return (n + na + i8_bn(S) - 1) / i8_bn(S); }
 int kbk_i8_rows(int S, int n, int na) { return kbk_i8_nrb(S, n, na) * i8_bn(S); }
 long long kbk_i8_total_tiles(int S, int n, int na, long long* tile_off /* [nrb+1] or null */) {
@@ -430,7 +455,7 @@ static cudaError_t i8_attr() {
 }
 cudaError_t kbk_solve_i8_init() {
 #define KB_ATTR(S) KB_CUDA_OK((i8_attr<S, 2>())); KB_CUDA_OK((i8_attr<S, 3>())); KB_CUDA_OK((i8_attr<S, KB_GEO>()));
-    KB_ATTR(4) KB_ATTR(5) KB_ATTR(6)
+    KB_ATTR(4) KB_ATTR(5) KB_ATTR(6) KB_ATTR(8)
 #undef KB_ATTR
     return cudaSuccess;
 }
@@ -445,7 +470,8 @@ static cudaError_t i8_launch(int dim, const SolvePtParams& p, int grid, cudaStre
 }
 cudaError_t kbk_solve_i8(int S, int dim, const SolvePtParams& p, int grid, cudaStream_t st) {
     if (p.vg.model < KB200_VG_LINEAR || p.vg.model > KB200_VG_TABLE) return cudaErrorInvalidValue;
-    return S == 6 ? i8_launch<6>(dim, p, grid, st) : S == 5 ? i8_launch<5>(dim, p, grid, st) : i8_launch<4>(dim, p, grid, st);
+    return S == 8 ? i8_launch<8>(dim, p, grid, st) : S == 6 ? i8_launch<6>(dim, p, grid, st)
+         : S == 5 ? i8_launch<5>(dim, p, grid, st) : i8_launch<4>(dim, p, grid, st);
 }
 
 // W (+ dual rows) -> row scales + int8 slice tiles. tile_off_dev: device copy of the per-row-block tile offsets.
@@ -455,7 +481,8 @@ cudaError_t kbk_pack_i8(int S, const double* W, int ld, int n, int n_pad, int na
     int nrows = nrb * i8_bn(S);
     i8_rowscale_kernel<<<(nrows + 7) / 8, 256, 0, st>>>(W, ld, n, n_pad, na, Uz, nrows, rowexp, rowscale);
     dim3 grid(nk, nrb);
-    if (S == 6) i8_pack_kernel<6><<<grid, 256, 0, st>>>(W, ld, n, n_pad, na, Uz, rowexp, nk, tile_off_dev, (signed char*)out);
+    if (S == 8) i8_pack_kernel<8><<<grid, 256, 0, st>>>(W, ld, n, n_pad, na, Uz, rowexp, nk, tile_off_dev, (signed char*)out);
+    else if (S == 6) i8_pack_kernel<6><<<grid, 256, 0, st>>>(W, ld, n, n_pad, na, Uz, rowexp, nk, tile_off_dev, (signed char*)out);
     else if (S == 5) i8_pack_kernel<5><<<grid, 256, 0, st>>>(W, ld, n, n_pad, na, Uz, rowexp, nk, tile_off_dev, (signed char*)out);
     else i8_pack_kernel<4><<<grid, 256, 0, st>>>(W, ld, n, n_pad, na, Uz, rowexp, nk, tile_off_dev, (signed char*)out);
     return cudaGetLastError();
